@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port, torch-cpu)
+  python bench.py --steps K --warmup W --dump-outputs DIR  # also writes the last timed step's joints as DIR/coords3d_abs.npy
 
 One JSON line on rank 0.  `value`: whole-job crops/s with the crops already resident in HBM.  `e2e`: the same metric
 through the reference-facing host-buffer call (mtb_forward_host: pinned host crops -> H2D -> forward -> D2H joints).
@@ -22,6 +23,7 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 
 METRIC = 'crops/sec'
+DUMP_LIMIT_BYTES = 64e6  # --dump-outputs writes at most this much
 NAMES = {'s': 'efficientnetv2-s', 'm': 'efficientnetv2-m', 'l': 'efficientnetv2-l', 'tiny': 'efficientnetv2-tiny',
          'resnet50': 'resnet50', 'mobilenetv3-small': 'mobilenetv3-small'}
 
@@ -29,7 +31,9 @@ NAMES = {'s': 'efficientnetv2-s', 'm': 'efficientnetv2-m', 'l': 'efficientnetv2-
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=10,
+                    help='timed steps of `value`, `e2e`, the graph replay and --impl reference (the tf32x3 sibling line runs '
+                         'min(steps, 5); the frames leg and the CPU baseline run fixed counts)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--size', default='l', choices=list(NAMES))
@@ -48,7 +52,15 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--graph', type=int, default=int(os.environ.get('MTB_BENCH_GRAPH', '0')),
                     help='1: replay the forward from a CUDA graph in the `value` region (mtb_forward never syncs or allocates)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the joints of the last timed step to DIR/coords3d_abs.npy (float32), to compare two builds '
+                         'output for output (the inputs and weights are seeded, so the same arguments give the same inputs)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes what the CUDA path computed: use it with --impl b200')
+    return args
 
 
 def peaks():
@@ -225,7 +237,7 @@ def best_thread_count(args, sd, spec, pcfg, probe_crops=4):
 
 def cpu_reference_forward(args, n_crops, iters, warmup, setup=None):
     """The reference's CPU path (oracle port of metrabs_pytorch Metrabs.forward, torch-cpu fp32, all usable host threads) on
-    `n_crops` synthetic crops per iteration, in chunks of <= 32 crops; 2 warm-ups + >= 5 timed iterations, median
+    `n_crops` synthetic crops per iteration, in chunks of <= 32 crops; `warmup` warm-ups + `iters` timed iterations, median
     (BASELINE.md section 2).  -> (crops/s, threads, median seconds per iteration, description dict)."""
     from oracle import port
     sd, spec, pcfg = setup or oracle_setup(args)
@@ -258,7 +270,7 @@ def run_reference(args):
     if rank != 0:
         return
     n = args.cpu_sample
-    v, cores, sec, desc = cpu_reference_forward(args, n, max(args.steps, 5), 2)
+    v, cores, sec, desc = cpu_reference_forward(args, n, args.steps, args.warmup)
     line = {
         'impl': 'reference', 'metric': METRIC, 'value': v, 'unit': 'crops/s', 'n_gpus': args.gpus,
         'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': sec * 1e3, 'higher_is_better': True,
@@ -410,6 +422,8 @@ def time_mode(args, eng, world, rank, device, dist, sharded_inputs):
     elapsed_ms = ev0.elapsed_time(ev1)
     prof_dom = eng.profile_end()[dom_name]
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
+    # the legs below reuse out_d: keep what the last timed step returned
+    last_out = out_d.cpu() if args.dump_outputs else None
 
     # ---- end to end through the host-buffer entry points: pinned host crops in, host joints out, EVERY step
     e2e_ms, e2e_mode = None, None
@@ -465,7 +479,7 @@ def time_mode(args, eng, world, rank, device, dist, sharded_inputs):
         e2e_ms = (time.perf_counter() - t0) * 1e3
         e2e_mode = 'per step: H2D local crops + intrinsics, mtb_forward_sharded (one NCCL all-gather), D2H full joints, sync'
     return dict(elapsed_ms=elapsed_ms, launches=launches, prof_all=prof_all, prof_dom=prof_dom, dom_name=dom_name, clocks=clocks,
-                e2e_ms=e2e_ms, e2e_mode=e2e_mode, graph_ms=graph_ms)
+                e2e_ms=e2e_ms, e2e_mode=e2e_mode, graph_ms=graph_ms, last_out=last_out)
 
 
 def run_b200(args):
@@ -488,6 +502,8 @@ def run_b200(args):
     else:
         B = args.batch            # per-GPU work fixed
     B_total = B * world
+    if args.dump_outputs and B_total * J * 3 * 4 > DUMP_LIMIT_BYTES:
+        raise SystemExit(f'--dump-outputs: {B_total} x {J} x 3 float32 joints exceed {DUMP_LIMIT_BYTES / 1e6:.0f} MB')
 
     def make_engine(precision):
         a = argparse.Namespace(**vars(args))
@@ -542,6 +558,10 @@ def run_b200(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:  # [B_total, J, 3] absolute camera-space joints (mm), the full batch on every rank
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, 'coords3d_abs.npy'), r['last_out'].numpy().astype(np.float32))
     pk = peaks()
     value = B_total * args.steps / (elapsed_ms / 1e3)
     e2e = B_total * args.steps / (e2e_ms / 1e3)

@@ -25,6 +25,14 @@ OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 
 JOINT_NAMES = ['pelv', 'lhip', 'rhip', 'lkne', 'rkne', 'neck', 'lsho', 'rsho']
 JOINT_EDGES = [(0, 1), (0, 2), (1, 3), (2, 4), (0, 5), (5, 6), (5, 7)]
 MIRROR = [0, 2, 1, 4, 3, 5, 7, 6]
+CROP_SAMPLE = 16  # one pixel in 16 of each crop batch is stored: the whole batches would put the fixture over 1 MB
+
+
+def pixel_sample(crops, seed):
+    """(sorted flat indices, values) of a fixed, seeded sample of 1/CROP_SAMPLE of the elements of ``crops``."""
+    flat = crops.reshape(-1).numpy()
+    idx = np.sort(np.random.default_rng(seed).choice(flat.size, flat.size // CROP_SAMPLE, replace=False)).astype(np.int32)
+    return idx, flat[idx]
 
 
 class StubJointInfo:
@@ -136,7 +144,7 @@ def main():
             for af in (1, 2):
                 crops, new_k, rot = est._get_crops(imgs_lin, k_box, d_box, cam_up, torch.cat(boxes), image_ids, rf, sc, gam, af)
                 tag = f'crops_a{num_aug}_af{af}'
-                data[tag] = crops.reshape(-1, 3, 64, 64).numpy()
+                data[tag + '_idx'], data[tag] = pixel_sample(crops.reshape(-1, 3, 64, 64), seed=10 * num_aug + af)
                 data[tag + '_newk'] = new_k.numpy()
                 data[tag + '_rot'] = rot.numpy()
                 invp = torch.linalg.inv(new_k @ rot)  # the reference's own fp32 inverse (multiperson_model.py:288, :292-295)

@@ -45,6 +45,8 @@ def test_joint_info_mirror():
 
 def test_golden_files_present(golden_dir):
     g = np.load(os.path.join(golden_dir, 'multiperson_pipeline.npz'), allow_pickle=False)
-    assert g['crops_a5_af1'].shape == (25, 3, 64, 64) and g['images'].dtype == np.uint8
+    idx = g['crops_a5_af1_idx']  # a sample of the pixels of the 25 crops [25, 3, 64, 64], touching every crop
+    assert g['crops_a5_af1'].shape == idx.shape and 0 <= idx.min() and idx.max() < 25 * 3 * 64 * 64
+    assert len(np.unique(idx // (3 * 64 * 64))) == 25 and g['images'].dtype == np.uint8
     f = np.load(os.path.join(golden_dir, 'multiperson_filter.npz'), allow_pickle=False)
     assert f['keep'].sum() > 0
