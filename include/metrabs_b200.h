@@ -289,6 +289,14 @@ int mtb_debug_run_op(mtb_handle* h, int op_index, const float* in, const float* 
 int mtb_op_is_fused_block(const mtb_handle* h, int op_index);
 int mtb_debug_run_fused_block(mtb_handle* h, int op_index, const float* in, int batch, float* out, size_t out_floats,
                               void* workspace, size_t workspace_bytes, void* stream);
+/* MBConv front-half fusion (bf16 tensor-core mode, 16x16 and 8x8 maps): 1 when backbone op `op_index` (a 1x1 stride-1 expand
+ * conv + SiLU) and the op after it (depthwise 3x3 stride 1 + SiLU, squeeze-excitation squeeze) run as ONE expdw_kernel launch
+ * (reference block: metrabs_pytorch/backbones/efficientnet.py:110-173).  mtb_debug_run_expdw runs that pair in isolation on a
+ * caller-provided fp32 NHWC device tensor `in` [B,H,W,Cin], fused (fused != 0) or as the two launches of the unfused path;
+ * `out` receives the depthwise output [B,H,W,Cexp] and `pooled` the squeeze-excitation means [B,Cexp], both fp32. */
+int mtb_op_is_expdw(const mtb_handle* h, int op_index);
+int mtb_debug_run_expdw(mtb_handle* h, int op_index, const float* in, int batch, float* out, size_t out_floats, float* pooled,
+                        size_t pooled_floats, int fused, void* workspace, size_t workspace_bytes, void* stream);
 /* CUDA-event profiler (bench.py's live roofline measurement): between begin and end, every kernel launch of the
  * classes selected by `class_mask` (bit i = class i) is bracketed by cudaEventRecord on the launching stream.
  * mtb_profile_end synchronises those events and returns, per class, the summed device time (ms), algorithmic
@@ -315,6 +323,10 @@ int mtb_debug_dw_plan(int height, int width, int* crops_per_item, int* rows_per_
  * plan for a block shape (all outputs 0 when the shape is not covered) and the stage images of the two weight matrices
  * (w1 [cexp][9*cin], w2 [cout][cexp], any 16-bit element type; pair = 1: the half-per-CTA images of the cta_group::2 kernel). */
 int mtb_debug_fmb_plan(int cin, int cexp, int cout, int pair, int* nstages, int* npatch, int* stage_bytes, int* smem_bytes);
+/* Host-side plan of the fused expand + depthwise kernel for an (H, W, Cin, Cexp) block shape (no device needed): pixels and
+ * crops per tile, weight ring stages and dynamic shared-memory bytes; all 0 when the shape keeps the two launches. */
+int mtb_debug_expdw_plan(int height, int width, int cin, int cexp, int* pixels_per_tile, int* crops_per_tile, int* nstages,
+                         int* smem_bytes);
 int mtb_debug_fmb_pack(const uint16_t* w1, const uint16_t* w2, int cin, int cexp, int cout, int pair, uint16_t* img1, uint16_t* img2);
 
 #ifdef __cplusplus

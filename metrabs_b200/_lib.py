@@ -111,6 +111,9 @@ _SIGNATURES = {
     'mtb_op_is_fused_block': (C.c_int, [C.c_void_p, C.c_int]),
     'mtb_debug_run_fused_block': (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
                                             C.c_size_t, C.c_void_p]),
+    'mtb_op_is_expdw': (C.c_int, [C.c_void_p, C.c_int]),
+    'mtb_debug_run_expdw': (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                      C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     'mtb_profile_begin': (C.c_int, [C.c_void_p, C.c_uint]),
     'mtb_profile_end': (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double),
                                   C.POINTER(C.c_int64)]),
@@ -125,6 +128,8 @@ _SIGNATURES = {
                                     C.POINTER(C.c_int)]),
     'mtb_debug_fmb_plan': (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
                                      C.POINTER(C.c_int)]),
+    'mtb_debug_expdw_plan': (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                       C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     'mtb_debug_fmb_pack': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
 }
 

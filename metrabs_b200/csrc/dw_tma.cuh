@@ -100,6 +100,102 @@ __device__ __forceinline__ f32x2 f2_act(f32x2 x) {
   }
 }
 
+// n 32-bit words from / to shared or global memory as one vector access (n = 1, 2 or 4)
+template <int N>
+__device__ __forceinline__ void ld_words(const void* a, unsigned (&wd)[N]) {
+  if constexpr (N == 4) { const uint4 r = *reinterpret_cast<const uint4*>(a); wd[0] = r.x; wd[1] = r.y; wd[2] = r.z; wd[3] = r.w; }
+  else if constexpr (N == 2) { const uint2 r = *reinterpret_cast<const uint2*>(a); wd[0] = r.x; wd[1] = r.y; }
+  else { wd[0] = *reinterpret_cast<const unsigned*>(a); }
+}
+template <int N>
+__device__ __forceinline__ void st_words(void* a, const unsigned (&wd)[N]) {
+  if constexpr (N == 4) *reinterpret_cast<uint4*>(a) = make_uint4(wd[0], wd[1], wd[2], wd[3]);
+  else if constexpr (N == 2) *reinterpret_cast<uint2*>(a) = make_uint2(wd[0], wd[1]);
+  else *reinterpret_cast<unsigned*>(a) = wd[0];
+}
+
+// One strip of the depthwise 3x3 stride-1 conv: rows_run (<= DWT_RUN) output rows x DWT_OW output columns x 2*NV channels,
+// row-input-stationary (each of the rows_run + 2 input rows is read and unpacked once and updates the three output rows it
+// feeds).  Every output starts its FMA chain from the bias and takes the taps in row-major order; then activation, store, and
+// the activated fp32 values are added to psum in row-major order.  Shared by dw3x3s1_tma_kernel and expdw_kernel, so that
+// both compute every output and every strip sum the same way.
+//   patch: 128-byte pixel rows, PW pixels per patch row; pix0 = patch pixel of the strip's top-left input;
+//   cbyte: byte offset of this thread's channels inside a pixel row; SWZ: 16-byte chunk k of patch pixel x sits at chunk
+//   position k ^ (x & 7) (expdw_kernel: its TMEM-lane = pixel stores are bank-conflict free that way);
+//   ncols: valid output columns of the strip; obase: output of (first row, first column, first channel).
+template <int ACT, typename T, int NV, bool SWZ>
+__device__ __forceinline__ void dw_strip(const uint8_t* patch, int pix0, int PW, int cbyte, int rows_run, int ncols, T* obase,
+                                         size_t row_stride, size_t px_stride, const f32x2 (&w)[9][NV], const f32x2 (&bias)[NV],
+                                         f32x2 (&psum)[NV]) {
+  constexpr bool F32 = sizeof(T) == 4;
+  constexpr int NW = F32 ? 2 * NV : NV;  // 32-bit words per pixel of this thread
+  f32x2 acc[3][DWT_OW][NV];
+#pragma unroll
+  for (int pr = 0; pr < DWT_RUN + 2; ++pr) {
+    if (pr < rows_run + 2) {
+      // input row pr of the run is tap row r of output row pr - r (slot (pr - r) % 3); the first tap of an output row
+      // (r = 0, s = 0) starts from the bias
+#pragma unroll
+      for (int x = 0; x < DWT_OW + 2; ++x) {
+        const int pix = pix0 + pr * PW + x;
+        const int off = SWZ ? ((((cbyte >> 4) ^ (pix & 7)) << 4) | (cbyte & 15)) : cbyte;
+        unsigned wd[NW];
+        ld_words<NW>(patch + (size_t)pix * 128 + off, wd);
+        f32x2 v[NV];
+#pragma unroll
+        for (int k = 0; k < NV; ++k) {
+          if constexpr (F32) v[k] = f2_pack(__uint_as_float(wd[2 * k]), __uint_as_float(wd[2 * k + 1]));
+          else v[k] = f2_pack(__uint_as_float(wd[k] << 16), __uint_as_float(wd[k] & 0xffff0000u));
+        }
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+          const int o = pr - r;  // compile-time
+          if (o < 0 || o >= DWT_RUN) continue;
+#pragma unroll
+          for (int i = 0; i < DWT_OW; ++i) {
+            const int s_ = x - i;  // compile-time
+            if (s_ >= 0 && s_ < 3) {
+#pragma unroll
+              for (int k = 0; k < NV; ++k)
+                acc[o % 3][i][k] = f2_fma(v[k], w[r * 3 + s_][k], (r == 0 && s_ == 0) ? bias[k] : acc[o % 3][i][k]);
+            }
+          }
+        }
+      }
+      // output row pr - 2 is complete
+      if (pr >= 2 && pr - 2 < rows_run) {
+        const int o = pr - 2, slot = o % 3;
+        T* orow = obase + (size_t)o * row_stride;
+#pragma unroll
+        for (int i = 0; i < DWT_OW; ++i) {
+          if (i < ncols) {
+            unsigned ov[NW];
+#pragma unroll
+            for (int k = 0; k < NV; ++k) {
+              if constexpr (F32) {
+                float x0, x1;
+                f2_unpack(acc[slot][i][k], x0, x1);
+                const float a0 = act_t<ACT>(x0), a1 = act_t<ACT>(x1);  // exact activation: this is the parity mode
+                psum[k] = f2_add(psum[k], f2_pack(a0, a1));
+                ov[2 * k] = __float_as_uint(a0);
+                ov[2 * k + 1] = __float_as_uint(a1);
+              } else {
+                const f32x2 a = f2_act<ACT>(acc[slot][i][k]);
+                float a0, a1;
+                f2_unpack(a, a0, a1);
+                const __nv_bfloat162 b2 = __floats2bfloat162_rn(a0, a1);
+                ov[k] = *reinterpret_cast<const unsigned*>(&b2);
+                psum[k] = f2_add(psum[k], a);
+              }
+            }
+            st_words<NW>(orow + (size_t)i * px_stride, ov);
+          }
+        }
+      }
+    }
+  }
+}
+
 // T = __nv_bfloat16: 64 channels per item, 8 per thread (4 fp32 pairs), tanh.approx SiLU (the throughput mode);
 // T = float (the 3xTF32 parity mode): 32 channels per item, 4 per thread (2 pairs), EXACT activation, fp32 in and out.
 // Either way a pixel is 128 bytes of shared memory, so the tiling plan, the strips and the stages are the same.
@@ -178,7 +274,7 @@ dw3x3s1_tma_kernel(const __grid_constant__ CUtensorMap tmIn, const DwTmaParams p
       for (int g = own_g0; g < p.G; g += GSTEP) blocksum[g][own_ch] = 0.f;
     }
     mbar_wait(&full[stage], (uint32_t)((li >> 1) & 1));
-    const uint8_t* patch = smem + (size_t)stage * p.stage_bytes + j * 16;
+    const uint8_t* patch = smem + (size_t)stage * p.stage_bytes;
 
     for (int s0 = 0; s0 < p.nstrips; s0 += 16) {
       const int s = s0 + sidx;
@@ -194,77 +290,9 @@ dw3x3s1_tma_kernel(const __grid_constant__ CUtensorMap tmIn, const DwTmaParams p
         const int orow0 = band * DWT_RUN;                       // first output row of the run, relative to the item
         const int rows_run = min(DWT_RUN, rows_item - orow0);   // >= 1 by construction of `bands`
         if (b < p.B && rows_run > 0) {
-          const uint8_t* prow = patch + (size_t)((g * PHB + orow0) * PW + ow0) * 128;
           T* obase = reinterpret_cast<T*>(p.out) + ((size_t)(b * p.H + row0 + orow0) * p.W + ow0) * p.C + c;
-          f32x2 acc[3][DWT_OW][NV];
-#pragma unroll
-          for (int pr = 0; pr < DWT_RUN + 2; ++pr) {
-            if (pr < rows_run + 2) {
-              // one input row of the run (OW + 2 pixels x 8 channels, each read and unpacked once); it is tap row r of output
-              // row pr - r (slot (pr - r) % 3); the first tap of an output row (r = 0, s = 0) starts from the bias
-#pragma unroll
-              for (int x = 0; x < DWT_OW + 2; ++x) {
-                const uint4 raw = *reinterpret_cast<const uint4*>(prow + (size_t)(pr * PW + x) * 128);
-                const unsigned wd[4] = {raw.x, raw.y, raw.z, raw.w};
-                f32x2 v[NV];
-                if constexpr (F32) {
-                  v[0] = f2_pack(__uint_as_float(wd[0]), __uint_as_float(wd[1]));
-                  v[1] = f2_pack(__uint_as_float(wd[2]), __uint_as_float(wd[3]));
-                } else {
-#pragma unroll
-                  for (int k = 0; k < NV; ++k) v[k] = f2_pack(__uint_as_float(wd[k] << 16), __uint_as_float(wd[k] & 0xffff0000u));
-                }
-#pragma unroll
-                for (int r = 0; r < 3; ++r) {
-                  const int o = pr - r;  // compile-time
-                  if (o < 0 || o >= DWT_RUN) continue;
-#pragma unroll
-                  for (int i = 0; i < DWT_OW; ++i) {
-                    const int s_ = x - i;  // compile-time
-                    if (s_ >= 0 && s_ < 3) {
-#pragma unroll
-                      for (int k = 0; k < NV; ++k)
-                        acc[o % 3][i][k] = f2_fma(v[k], w[r * 3 + s_][k], (r == 0 && s_ == 0) ? bias[k] : acc[o % 3][i][k]);
-                    }
-                  }
-                }
-              }
-              // output row pr - 2 is complete
-              if (pr >= 2 && pr - 2 < rows_run) {
-                const int o = pr - 2, slot = o % 3;
-                T* orow = obase + (size_t)o * p.W * p.C;
-#pragma unroll
-                for (int i = 0; i < DWT_OW; ++i) {
-                  if (ow0 + i < p.W) {
-                    if constexpr (F32) {
-                      float a[4];
-#pragma unroll
-                      for (int k = 0; k < NV; ++k) {
-                        float x0, x1;
-                        f2_unpack(acc[slot][i][k], x0, x1);
-                        a[2 * k] = act_t<ACT>(x0);      // exact activation: this is the parity mode
-                        a[2 * k + 1] = act_t<ACT>(x1);
-                        psum[k] = f2_add(psum[k], f2_pack(a[2 * k], a[2 * k + 1]));
-                      }
-                      *reinterpret_cast<float4*>(orow + (size_t)i * p.C) = make_float4(a[0], a[1], a[2], a[3]);
-                    } else {
-                      uint4 ov;
-                      __nv_bfloat162* o2 = reinterpret_cast<__nv_bfloat162*>(&ov);
-#pragma unroll
-                      for (int k = 0; k < NV; ++k) {
-                        const f32x2 a = f2_act<ACT>(acc[slot][i][k]);
-                        float a0, a1;
-                        f2_unpack(a, a0, a1);
-                        o2[k] = __floats2bfloat162_rn(a0, a1);
-                        psum[k] = f2_add(psum[k], a);
-                      }
-                      *reinterpret_cast<uint4*>(orow + (size_t)i * p.C) = ov;
-                    }
-                  }
-                }
-              }
-            }
-          }
+          dw_strip<ACT, T, NV, false>(patch, (g * PHB + orow0) * PW + ow0, PW, j * 16, rows_run, p.W - ow0, obase, (size_t)p.W * p.C,
+                                      (size_t)p.C, w, bias, psum);
         }
       }
       if (p.pooled) {

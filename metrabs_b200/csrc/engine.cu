@@ -18,6 +18,7 @@
 #include "decode.cuh"
 #include "tc_gemm.cuh"
 #include "tc_fmb.cuh"
+#include "tc_expdw.cuh"
 #include "tc_tf32.cuh"
 #include "dw_tma.cuh"
 #include "multiperson.cuh"
@@ -32,11 +33,12 @@ enum OpType { OP_STEM = 0, OP_CONV = 1, OP_DW = 2, OP_POOL = 3, OP_MAXPOOL = 4 }
 // kernel classes for the CUDA-event profiler (mtb_profile_begin / mtb_profile_end)
 enum KClass { KC_STEM = 0, KC_IGEMM_SIMT = 1, KC_DWCONV = 2, KC_POOL = 3, KC_SE_FC = 4, KC_TC_GEMM = 5, KC_FMB = 6,
               KC_HEAD_FUSED = 7, KC_HEAD_CONV_SIMT = 8, KC_SOFTARGMAX = 9, KC_RECON = 10, KC_OTHER = 11, KC_SE_SCALE = 12, KC_TC32 = 13,
-              KC_COUNT = 14 };
+              KC_EXPDW = 14, KC_COUNT = 15 };
 const char* kKClassNames[KC_COUNT] = {"stem_conv_kernel", "conv_igemm_kernel", "dwconv_kernel", "pool_mean_kernel",
                                       "se_fc(conv_igemm_kernel)", "tc_conv_kernel", "fmb_kernel",
                                       "tc_head_softargmax_kernel", "head_conv(conv_igemm_kernel)",
-                                      "softargmax_bhwn_kernel", "recon_pass1+2_kernel", "other", "se_scale_kernel", "tc32_conv_kernel"};
+                                      "softargmax_bhwn_kernel", "recon_pass1+2_kernel", "other", "se_scale_kernel", "tc32_conv_kernel",
+                                      "expdw_kernel"};
 enum { BUF_FEATURES = -2, BUF_NONE = -1, BUF_SMALL0 = 4 };  // 0..3 big activation buffers, 4..6 small [B,C]
 constexpr int kNumBig = 4, kNumSmall = 3;
 constexpr int kPoolSlices = 8;  // the fused depthwise+pool kernel leaves up to 8 partial slices [slice][B][C]
@@ -71,6 +73,7 @@ struct Op {
   TcWeights tc;             // bf16 K-major copy + TMA descriptor state for the tcgen05 path
   Tc32Weights tc32;         // fp32 K-major copy + TMA descriptor state for the 3xTF32 tcgen05 path (MTB_PRECISION_TF32X3)
   FmbWeights fmb;           // bf16 mode: this 3x3 expand conv and the NEXT op (1x1 projection) run as one fmb_kernel launch
+  ExpdwWeights expdw;       // bf16 mode: this 1x1 expand conv and the NEXT op (depthwise 3x3 + SE squeeze) run as one expdw_kernel launch
   mutable DwTmaCache dw_cache;  // input tensor map of the TMA-staged depthwise kernel
   double flops = 0;         // 2*MACs per crop
   int stage = 0;            // EfficientNet stage (1-based; 0 = stem / last conv / other backbones)
@@ -718,6 +721,18 @@ int dw_pool_slices(const Op& dw, bool tma_ok = true) {
   return std::min((strips + 7) / 8, kPoolSlices);
 }
 
+// (a, d) = 1x1 expand + depthwise pair that expdw_kernel computes exactly as the two launches do (bf16 tensor-core mode;
+// the depthwise op runs dw3x3s1_tma_kernel with ONE pooled slice there, the layout the fused kernel writes)
+bool expdw_pair_ok(const mtb_handle* h, const Op& a, const Op& d) {
+  if (h->cfg.precision != MTB_PRECISION_BF16_TC || !a.tc.ready) return false;
+  if (a.type != OP_CONV || a.small_io || a.R != 1 || a.S != 1 || a.stride != 1 || a.act != ACT_SILU) return false;
+  if (a.res_buf != BUF_NONE || a.scale_buf != BUF_NONE || a.Hin != a.Hout || a.Win != a.Wout) return false;
+  if (d.type != OP_DW || d.act != ACT_SILU || !d.fused_pool || d.in_buf != a.out_buf || d.out_buf == a.in_buf || d.Cout != a.Cout) return false;
+  if (d.stride != 1 || d.pad_t != 1 || d.pad_l != 1 || d.Hout != a.Hout || d.Wout != a.Wout) return false;
+  const DwTmaPlan dp = dw_tma_plan_for(d);
+  return dp.ok && dp.n_rb == 1 && expdw_plan(a.Hout, a.Wout, a.Cin, a.Cout).ok;
+}
+
 int op_class(const Op& op) {
   switch (op.type) {
     case OP_STEM: return KC_STEM;
@@ -728,6 +743,7 @@ int op_class(const Op& op) {
   }
   if (op.small_io) return KC_SE_FC;
   if (op.fmb.ready && fmb_enabled()) return KC_FMB;
+  if (op.expdw.ready && expdw_enabled()) return KC_EXPDW;
   if (op.tc.ready) return KC_TC_GEMM;  // one class per kernel: every tensor-core conv/GEMM launch is tc_conv_kernel
   if (op.tc32.ready) return KC_TC32;
   return KC_IGEMM_SIMT;
@@ -928,6 +944,21 @@ int run_fused_block(mtb_handle* h, const Op& a, const Op& b, int B, const Worksp
   return MTB_OK;
 }
 
+// one expdw_kernel launch for the MBConv front half (a = 1x1 expand + SiLU, d = depthwise 3x3 + SiLU + SE squeeze into the
+// pooled buffer that fc1 reads, exactly as d's own launch leaves it)
+int run_expdw(mtb_handle* h, const Op& a, const Op& d, int B, const Workspace& ws, void* features, cudaStream_t st) {
+  const void* in = act_ptr(h, ws, a.in_buf, features, a.Hin, a.Win, a.Cin);
+  void* out = act_ptr(h, ws, d.out_buf, features, d.Hout, d.Wout, d.Cout);
+  float* pooled = (float*)buf_ptr(ws, BUF_SMALL0, features);
+  // algorithmic bytes: input + depthwise output + expand weights (bf16) + depthwise weights and both biases (fp32) + means
+  const double bytes = 2.0 * B * a.Hin * a.Win * (a.Cin + d.Cout) + 2.0 * a.Cin * a.Cout + 4.0 * 11.0 * a.Cout + 4.0 * B * d.Cout;
+  ProfScope prof(h, KC_EXPDW, (a.flops + d.flops) * B, bytes, st);
+  const char* e = expdw_launch(a.expdw, in, out, pooled, B, st);
+  if (e) return fail(h, MTB_ERR_CUDA, "fused expand + depthwise launch %s: %s", a.name.c_str(), e);
+  h->launches++;
+  return MTB_OK;
+}
+
 // ops [first, last): fusable pairs that lie inside the range run fused
 int run_ops_range(mtb_handle* h, size_t first, size_t last, const float* crops, int B, const Workspace& ws, void* features,
                   cudaStream_t st) {
@@ -937,6 +968,9 @@ int run_ops_range(mtb_handle* h, size_t first, size_t last, const float* crops, 
     if (h->ops[k].fmb.ready && fmb_enabled() && k + 1 < last) {
       rc = run_fused_block(h, h->ops[k], h->ops[k + 1], B, ws, features, st);
       ++k;
+    } else if (h->ops[k].expdw.ready && expdw_enabled() && k + 1 < last) {
+      rc = run_expdw(h, h->ops[k], h->ops[k + 1], B, ws, features, st);
+      ++k;  // the depthwise op; its OP_POOL successor is skipped as after the depthwise launch (fused_pool)
     } else {
       rc = run_op(h, h->ops[k], crops, B, ws, features, st);
     }
@@ -1255,6 +1289,16 @@ int mtb_finalize_weights(mtb_handle* h) {
     if (a.Hin != a.Hout || a.Win != a.Wout || b.out_buf == a.in_buf) continue;
     const char* e = fmb_prepare(a.fmb, a.tc, b.tc, h->dev_allocs);
     if (e) return fail(h, MTB_ERR_CUDA, "fused FusedMBConv weight prep for '%s': %s", a.name.c_str(), e);
+  }
+  // MBConv front halves (1x1 expand + SiLU -> depthwise 3x3 stride 1 + SiLU + SE squeeze) on 16x16 / 8x8 maps: one fused
+  // kernel per block (tc_expdw.cuh); every other shape keeps the two launches
+  for (size_t i = 0; i + 1 < h->ops.size(); ++i) {
+    Op& a = h->ops[i];
+    const Op& d = h->ops[i + 1];
+    a.expdw.ready = false;
+    if (!expdw_pair_ok(h, a, d)) continue;
+    const char* e = expdw_prepare(a.expdw, a.tc, d.d_w, d.d_bias, a.Hout, a.Wout);
+    if (e) return fail(h, MTB_ERR_CUDA, "fused expand + depthwise prep for '%s': %s", a.name.c_str(), e);
   }
   {
     Op& hd = h->head;
@@ -2005,6 +2049,52 @@ int mtb_debug_fmb_plan(int cin, int cexp, int cout, int pair, int* nstages, int*
 int mtb_debug_fmb_pack(const uint16_t* w1, const uint16_t* w2, int cin, int cexp, int cout, int pair, uint16_t* img1, uint16_t* img2) {
   if (!w1 || !w2 || !img1 || !img2 || !fmb_shape_ok(cin, cexp, cout)) return fail(nullptr, MTB_ERR_INVALID_ARG, "invalid arguments");
   fmb_pack_images(w1, w2, cin, cexp, cout, pair ? 2 : 1, img1, img2);
+  return MTB_OK;
+}
+
+int mtb_op_is_expdw(const mtb_handle* h, int op_index) {
+  return (h && op_index >= 0 && op_index + 1 < (int)h->ops.size() && h->ops[op_index].expdw.ready && expdw_enabled()) ? 1 : 0;
+}
+
+int mtb_debug_run_expdw(mtb_handle* h, int op_index, const float* in, int batch, float* out, size_t out_floats, float* pooled,
+                        size_t pooled_floats, int fused, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_common(h, batch, workspace_bytes, workspace);
+  if (rc) return rc;
+  if (op_index < 0 || op_index + 1 >= (int)h->ops.size() || !in || !out || !pooled) return fail(h, MTB_ERR_INVALID_ARG, "invalid debug arguments");
+  if (!h->ops[op_index].expdw.ready) return fail(h, MTB_ERR_UNSUPPORTED, "op %d does not start a fused expand + depthwise pair", op_index);
+  DeviceGuard g(h->cfg.device);
+  cudaStream_t st = (cudaStream_t)stream;
+  Workspace ws = layout(h, batch, workspace);
+  Op a = h->ops[op_index], d = h->ops[op_index + 1];  // copies with overridden buffers and fresh tensor-map caches
+  const size_t n_in = (size_t)batch * a.Hin * a.Win * a.Cin, n_out = (size_t)batch * d.Hout * d.Wout * d.Cout;
+  const size_t n_pool = (size_t)batch * d.Cout;
+  if (n_out > out_floats || n_pool > pooled_floats) return fail(h, MTB_ERR_INVALID_ARG, "debug output buffer too small");
+  launch_k(from_float_kernel, dim3(grid_for(n_in, 256)), dim3(256), 0, st, in, (__nv_bfloat16*)buf_ptr(ws, 0, nullptr), n_in);
+  a.in_buf = 0; a.out_buf = 1; d.in_buf = 1; d.out_buf = 2;
+  a.expdw.cached_in = nullptr;
+  a.tc.cached_in = nullptr;
+  a.tc.map_sets.clear();
+  d.dw_cache = DwTmaCache();
+  if (fused) {
+    rc = run_expdw(h, a, d, batch, ws, nullptr, st);
+  } else {  // the two launches, the depthwise one pooling as in a forward
+    rc = run_op(h, a, nullptr, batch, ws, nullptr, st);
+    if (!rc) rc = run_op(h, d, nullptr, batch, ws, nullptr, st);
+  }
+  if (rc) return rc;
+  launch_k(to_float_kernel, dim3(grid_for(n_out, 256)), dim3(256), 0, st, (const __nv_bfloat16*)buf_ptr(ws, 2, nullptr), out, n_out);
+  CUDA_TRY(h, cudaMemcpyAsync(pooled, buf_ptr(ws, BUF_SMALL0, nullptr), n_pool * 4, cudaMemcpyDeviceToDevice, st));
+  return MTB_OK;
+}
+
+int mtb_debug_expdw_plan(int height, int width, int cin, int cexp, int* pixels_per_tile, int* crops_per_tile, int* nstages,
+                         int* smem_bytes) {
+  if (!pixels_per_tile || !crops_per_tile || !nstages || !smem_bytes) return fail(nullptr, MTB_ERR_INVALID_ARG, "invalid arguments");
+  const ExpdwPlan pl = expdw_plan(height, width, cin, cexp);
+  *pixels_per_tile = pl.ok ? pl.pixels : 0;
+  *crops_per_tile = pl.ok ? pl.crops : 0;
+  *nstages = pl.ok ? pl.nstages : 0;
+  *smem_bytes = pl.ok ? pl.smem_bytes : 0;
   return MTB_OK;
 }
 

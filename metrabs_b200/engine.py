@@ -296,6 +296,24 @@ class Engine:
                                               ws.numel(), _stream_ptr(self.device)), self._h)
         return out
 
+    def op_is_expdw(self, op):
+        """True when backbone op `op` (1x1 expand) and op + 1 (depthwise 3x3 + SE squeeze) run as one expdw_kernel launch."""
+        return bool(lib().mtb_op_is_expdw(self._h, op))
+
+    def debug_run_expdw(self, op, x, fused=True):
+        """The expand + depthwise pair starting at op `op` in isolation, fused or as the two launches: x [B,H,W,Cin] fp32.
+        Returns (depthwise output [B,H,W,Cexp], squeeze-excitation means [B,Cexp]), both fp32."""
+        io = self.op_io(op + 1)
+        b = x.shape[0]
+        out = torch.empty((b,) + io['out_shape'], dtype=torch.float32, device=self.device)
+        pooled = torch.empty((b, io['out_shape'][-1]), dtype=torch.float32, device=self.device)
+        ws = self.workspace(b)
+        x = x.float().contiguous()
+        check(lib().mtb_debug_run_expdw(self._h, op, x.data_ptr(), b, out.data_ptr(), out.numel(), pooled.data_ptr(),
+                                        pooled.numel(), 1 if fused else 0, ws.data_ptr(), ws.numel(),
+                                        _stream_ptr(self.device)), self._h)
+        return out, pooled
+
     def profile_begin(self, classes=None):
         """Brackets every launch of the selected kernel classes (None = all) with CUDA events on the launch stream."""
         n = lib().mtb_num_kernel_classes()
